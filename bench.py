@@ -12,6 +12,8 @@ A "step" is one `PGTFormer.forward` over `--clips` synthetic 3-frame 512x512 cli
   cpu_baseline  the CPU oracle (port of the reference's PyTorch path) on the host cores, N=1 rank 0 only
 `--impl reference` times that CPU path alone (the reference has no CUDA code of its own and cannot
 travel to the GPU box; `oracle/pgt_oracle.py` is pinned to it by tests/golden/).
+`--dump-outputs DIR` writes what the last timed step computed, from inputs that are the same on every run, so two
+builds can be compared output for output.
 """
 import argparse
 import json
@@ -207,6 +209,27 @@ def north_star_kernels(b, H, dev, peaks):
     return res
 
 
+DUMP_MAX_ELEMENTS = 4 << 20            # per array: three fp32 arrays stay under 64 MB
+
+
+def dump_outputs(outputs, directory):
+    """Writes each output as <directory>/<name>.npy in float32.  An output with more than DUMP_MAX_ELEMENTS elements is
+    replaced by the elements at a fixed seeded sample of flat indices (sorted; the same for every run of one shape), so
+    two builds can be compared output for output.  Returns {name: {'shape', 'stored', 'sampled'}}."""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    info = {}
+    for name, t in outputs.items():
+        stored = t
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            idx = torch.randint(t.numel(), (DUMP_MAX_ELEMENTS,), generator=torch.Generator().manual_seed(0))
+            stored = t.reshape(-1)[idx.sort().values.to(t.device)]
+        np.save(os.path.join(directory, name + '.npy'), stored.float().cpu().numpy())
+        info[name] = {'shape': list(t.shape), 'stored': stored.numel(), 'sampled': stored is not t}
+    return info
+
+
 def run_reference(args):
     """`--impl reference`: the reference's own CPU implementation of the path (oracle port), host cores only."""
     rank = int(os.environ.get('RANK', '0'))
@@ -239,7 +262,13 @@ def main():
     ap.add_argument('--gather', default='middle_u8', choices=['middle_u8', 'full'],
                     help='N > 1: what the end-of-step all-gather carries (restored middle frames as rgb24, or every fp32 frame)')
     ap.add_argument('--no-parity', action='store_true', help='skip the golden-vector parity block of the JSON line')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last timed step returned (out: the step result, '
+                         'logits, lq_feat) as DIR/<name>.npy in float32; arrays over %d elements as a fixed seeded '
+                         'sample' % DUMP_MAX_ELEMENTS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         return run_reference(args)
 
@@ -277,8 +306,12 @@ def main():
             return out
         return gather_frames(out, world * b) if args.gather == 'full' else gather_restored(out, world * b)
 
+    last = {}
+
     def step_resident():
-        return collective(model(x_dev, w=1, adain=True)[0])
+        out, last['logits'], last['lq_feat'] = model(x_dev, w=1, adain=True)
+        last['out'] = collective(out)
+        return last['out']
 
     # end to end as a serving loop would run it: the pinned-host -> device copy of step k+1 and the device -> host copy
     # of step k's result ride their own streams and overlap the compute of the neighbouring step; every step still does
@@ -342,6 +375,8 @@ def main():
     launches = ops.launch_count() if not args.graph else launches_per_forward * args.steps
     clocks = sampler.stop() if rank == 0 else None
     value = world * b * args.steps / (ms / 1000.0)
+    # before the e2e pass: with --graph the outputs are static tensors the next replay rewrites
+    dumped = dump_outputs(last, args.dump_outputs) if rank == 0 and args.dump_outputs else None
 
     for _ in range(2):
         step_e2e()
@@ -395,6 +430,8 @@ def main():
             'north_star_kernels': ns_kernels,
             'parity': parity,
         }
+        if dumped is not None:
+            line['dumped_outputs'] = {'dir': args.dump_outputs, 'arrays': dumped}
         tr = load_traffic()
         if tr is not None:
             line['roofline']['traffic'] = tr.get('dram_bytes_per_launch')

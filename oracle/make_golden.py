@@ -7,6 +7,8 @@ Run in the build container (the reference does not exist on the GPU box):
     python -m oracle.make_golden --full     # 512^2 (the reference's native size, NO size patch) and 1024^2 (size patch)
     python -m oracle.make_golden --video    # first 8 frames of assets/inputdemovideo.mp4 through inference.py's loop
     python -m oracle.make_golden --swin     # the Video-Swin BasicLayer of modules/swin.py (TDRQVAE) on stand-in weights
+    python -m oracle.make_golden --tiny     # 64^2 (strided sample of every output)
+    python -m oracle.make_golden --swin-spec --checkpoint   # BasicLayer state-dict layout; save_pretrained layout
 Inputs are not stored: `golden_input(seed, b, H)` regenerates them bit-exactly.
 
 The full-size fixtures are stored compactly (the raw outputs are 50-200 MB): every code index (int16), the top-2
@@ -28,6 +30,7 @@ GOLDEN = os.path.join(ROOT, 'tests', 'golden')
 OPT = os.path.join(ROOT, 'options', 'release_test_stage_IIII_dont_need_align_version.yml')
 DEMO_VIDEO = 'assets/inputdemovideo.mp4'          # relative to the reference root
 N_LOGIT_ROWS = 384
+SAMPLE_STRIDE = 11
 
 
 def load_network_g():
@@ -155,16 +158,22 @@ def video(n=8):
     print('wrote %s in %.0f s (%.1f MB)' % (path, time.time() - t0, os.path.getsize(path) / 1e6), frames.shape, restored.shape)
 
 
-def swin():
-    """The reference's Video-Swin `BasicLayer` (`modules/swin.py:326-405`, imported with the mmcv / basicsr / timm shims)
-    on the deterministic stand-in weights of oracle/swin3d_oracle.py: outputs stored as fp16."""
+def _reference_swin_module():
+    """The reference's `modules/swin.py`, imported with the mmcv / basicsr / timm shims."""
     import importlib.util
-    from oracle import swin3d_oracle as S
     from oracle.reference_loader import REFERENCE_ROOT, _ensure_paths
     _ensure_paths()
     spec = importlib.util.spec_from_file_location('_pgt_reference.modules.swin', os.path.join(REFERENCE_ROOT, 'modules', 'swin.py'))
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
+    return mod
+
+
+def swin():
+    """The reference's Video-Swin `BasicLayer` (`modules/swin.py:326-405`, imported with the mmcv / basicsr / timm shims)
+    on the deterministic stand-in weights of oracle/swin3d_oracle.py: outputs stored as fp16."""
+    from oracle import swin3d_oracle as S
+    mod = _reference_swin_module()
     for name, c in S.SWIN_CASES.items():
         layer = mod.BasicLayer(c['dim'], c['depth'], c['heads'], c['window']).eval()
         layer.load_state_dict(S.synth_state(layer.state_dict(), c['seed']), strict=True)
@@ -176,11 +185,63 @@ def swin():
         print('wrote', path, tuple(y.shape), '%.1f KB' % (os.path.getsize(path) / 1e3))
 
 
+def tiny(seed=7, H=64):
+    """The reference's forward at 64^2: every code index and every SAMPLE_STRIDE-th element of out, logits and
+    lq_feat (flattened, fp32).  The stride is prime, so the sample walks through every channel of the
+    power-of-two-wide tensors."""
+    from oracle.reference_loader import reference_forward
+    m = _reference_model()
+    out, logits, lq = reference_forward(m, golden_input(seed, 1, H), w=1.0, adain=True)
+    rec = {'seed': seed, 'b': 1, 'H': H, 'w': 1.0, 'adain': True, 'stride': SAMPLE_STRIDE,
+           'codes': logits.argmax(-1).to(torch.int16)}
+    for k, v in (('out', out), ('logits', logits), ('lq_feat', lq)):
+        rec[k] = v.reshape(-1)[::SAMPLE_STRIDE].clone()
+        rec[k + '_shape'] = list(v.shape)
+    path = os.path.join(GOLDEN, 'pgtformer_ref_b1_%d_seed%d_strided.pt' % (H, seed))
+    torch.save(rec, path)
+    print('wrote %s (%.1f KB)' % (path, os.path.getsize(path) / 1e3))
+
+
+def swin_spec():
+    """Parameter / buffer names, shapes and dtypes of the reference's `BasicLayer(256, 4, 8, (5, 5, 5))`, and its
+    relative_position_index (values < 729, stored as int16): the state-dict layout `modules/swin.py` reproduces."""
+    sd = _reference_swin_module().BasicLayer(256, 4, 8, (5, 5, 5)).state_dict()
+    path = os.path.join(GOLDEN, 'swin3d_basic_layer_state_spec.pt')
+    torch.save({'spec': {k: (list(v.shape), str(v.dtype)) for k, v in sd.items()},
+                'relative_position_index': sd['blocks.0.attn.relative_position_index'].to(torch.int16)}, path)
+    print('wrote %s: %d entries (%.1f KB)' % (path, len(sd), os.path.getsize(path) / 1e3))
+
+
+def checkpoint_layout():
+    """What the reference class's `save_pretrained` writes, the layout of a Hub checkpoint such as
+    kepeng/pgtformer-base: config.json and the model.safetensors header, both verbatim.  The 500 MB tensor payload is
+    not kept; the loader test fills the recorded offsets with seeded values."""
+    import gzip
+    import json
+    import struct
+    import tempfile
+    from oracle.reference_loader import build_reference_model
+    ref = build_reference_model(load_network_g())
+    with tempfile.TemporaryDirectory() as d:
+        ref.save_pretrained(d)
+        with open(os.path.join(d, 'config.json')) as f:
+            config = f.read()
+        with open(os.path.join(d, 'model.safetensors'), 'rb') as f:
+            header = f.read(struct.unpack('<Q', f.read(8))[0]).decode()
+    path = os.path.join(GOLDEN, 'reference_checkpoint_layout.json.gz')
+    with open(path, 'wb') as f, gzip.GzipFile(fileobj=f, mode='wb', mtime=0) as z:
+        z.write(json.dumps({'config.json': config, 'model.safetensors header': header}).encode())
+    print('wrote %s (%.1f KB)' % (path, os.path.getsize(path) / 1e3))
+
+
 if __name__ == '__main__':
     ap = argparse.ArgumentParser()
     ap.add_argument('--full', action='store_true')
     ap.add_argument('--video', action='store_true')
     ap.add_argument('--swin', action='store_true')
+    ap.add_argument('--tiny', action='store_true')
+    ap.add_argument('--swin-spec', action='store_true')
+    ap.add_argument('--checkpoint', action='store_true')
     a = ap.parse_args()
     if a.full:
         full()
@@ -188,5 +249,11 @@ if __name__ == '__main__':
         video()
     if a.swin:
         swin()
-    if not (a.full or a.video or a.swin):
+    if a.tiny:
+        tiny()
+    if a.swin_spec:
+        swin_spec()
+    if a.checkpoint:
+        checkpoint_layout()
+    if not (a.full or a.video or a.swin or a.tiny or a.swin_spec or a.checkpoint):
         small()

@@ -1,9 +1,11 @@
 """Checkpoint formats of the drop-in class (SURVEY 8f #3): HF `config.json + model.safetensors` directories
 (`PGTFormer.from_pretrained`, inference.py:118) and BasicSR `.pth` files with `params_ema` (inference_cn.py:124-126),
-including a directory written by the REFERENCE class itself when /root/reference is present."""
+including the layout of a directory written by the REFERENCE class itself."""
+import gzip
+import json
 import os
+import struct
 
-import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -54,18 +56,37 @@ def test_basicsr_params_ema_pth(network_g, tmp_path):
         assert torch.equal(v, want[k]), k
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/archs'), reason='reference tree not mounted')
-def test_directory_written_by_the_reference_class_loads(network_g, tmp_path):
-    """What `PGTFormer.from_pretrained("kepeng/pgtformer-base")` downloads is a directory the reference class wrote."""
+def test_directory_written_by_the_reference_class_loads(tmp_path):
+    """What `PGTFormer.from_pretrained("kepeng/pgtformer-base")` downloads is a directory the reference class wrote.
+    config.json and the model.safetensors header are the reference's own, byte for byte (oracle/make_golden.py
+    --checkpoint); the tensor payload at the recorded offsets is seeded, so a no-op load cannot pass."""
     from archs.pgtformer_arch import PGTFormer
-    from oracle import reference_loader as RL
-    ref = RL.build_reference_model(network_g)
-    ref.save_pretrained(str(tmp_path))
+    with gzip.open(os.path.join(ROOT, 'tests', 'golden', 'reference_checkpoint_layout.json.gz'), 'rt') as f:
+        layout = json.load(f)
+    (tmp_path / 'config.json').write_text(layout['config.json'])
+    header = layout['model.safetensors header'].encode()
+    entries = sorted(((k, v) for k, v in json.loads(header).items() if k != '__metadata__'),
+                     key=lambda kv: kv[1]['data_offsets'][0])
+    g = torch.Generator().manual_seed(11)
+    want = {}
+    with open(tmp_path / 'model.safetensors', 'wb') as f:
+        f.write(struct.pack('<Q', len(header)) + header)
+        pos = 0
+        for k, v in entries:
+            assert v['data_offsets'][0] == pos, k
+            if v['dtype'] == 'F32':
+                t = torch.randn(v['shape'], generator=g)
+            else:
+                assert v['dtype'] == 'I64', k
+                t = torch.randint(0, 1000, v['shape'], generator=g)
+            f.write(t.numpy().tobytes())
+            pos = v['data_offsets'][1]
+            want[k] = t
     ours = PGTFormer.from_pretrained(str(tmp_path))
-    rsd, osd = ref.state_dict(), ours.state_dict()
-    assert set(rsd) == set(osd) and len(osd) == 961        # registration order differs, names do not
-    for k in rsd:
-        assert torch.equal(rsd[k], osd[k]), k
+    osd = ours.state_dict()
+    assert set(want) == set(osd) and len(osd) == 961        # registration order differs, names do not
+    for k in want:
+        assert osd[k].dtype == want[k].dtype and torch.equal(osd[k], want[k]), k
 
 
 def test_submodule_load_and_refresh_drop_the_packed_engine(network_g):
